@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # native arm (one process per GPU under torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path, timed on the host cores (rank 0 only)
+    python bench.py ... --dump-outputs DIR                   # also write the samples of the last timed step to DIR/*.npy
 
 Workload (BASELINE.json configs[1]): EDM CIFAR-10 32x32 DDPM++ U-Net (random init, de-zeroed so |F_x| = O(1)), Heun sampler,
 num_steps=10 => NFE=18, batch 512 per GPU, synthetic Gaussian latents.  One "step" = one full sampling pass over one batch.
@@ -55,7 +56,12 @@ def parse():
     ap.add_argument('--all_configs', type=int, default=1, help='1 (default, N=1 only): also measure BASELINE configs 3-5 into `configs`')
     ap.add_argument('--config_steps', type=int, default=10, help='timed steps of each `configs` entry')
     ap.add_argument('--gpu_eager', type=int, default=1, help='1 (default, N=1 only): time the eager-PyTorch GPU path of the same configs')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last timed step returned (rank 0; each `configs` entry too) as DIR/<name>.npy in '
+                         f'float32, at most {DUMP_LIMIT_BYTES >> 20} MB in all')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.precision_requested = args.precision
     args.f8_min_channels_requested = args.f8_min_channels
     if args.precision == 'auto':
@@ -73,6 +79,25 @@ def peaks():
         return dict(hbm_gbs=d['hbm_gbs'], tflops_burst=d['bf16_tflops'], tflops_sustained=d.get('bf16_tflops_sustained', d['bf16_tflops']),
                     source='measured (MEASURED_PEAKS.json)')
     return dict(hbm_gbs=6650.0, tflops_burst=1590.0, tflops_sustained=1400.0, source='fallback (B200_PROFILING.md)')
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+    """`--dump-outputs`: every {name: tensor} as out_dir/<name>.npy in float32.  A run's inputs depend only on its arguments, so two builds
+    run with the same arguments can be compared file by file.  Over DUMP_LIMIT_BYTES in all, every array keeps the same fraction of its
+    leading (batch) rows, picked with a fixed seed, so the sample too is the same from run to run."""
+    import numpy as np
+    import torch
+    total = sum(t.numel() * 4 for t in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().to('cpu', torch.float32)
+        if total > DUMP_LIMIT_BYTES:
+            keep = t.shape[0] * DUMP_LIMIT_BYTES // total
+            t = t[torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(out_dir, name + '.npy'), t.numpy())
 
 
 class ClockSampler:
@@ -143,12 +168,12 @@ def cpu_reference_leg(args, steps, warmup):
     times = []
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        SO.sample(net, lat, args.solver, class_labels=lab, num_steps=args.num_steps)
+        samples = SO.sample(net, lat, args.solver, class_labels=lab, num_steps=args.num_steps)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
     tot = sum(times)
-    return dict(value=args.cpu_batch * len(times) / tot, seconds_per_step=tot / len(times), cores=cores,
+    return dict(value=args.cpu_batch * len(times) / tot, seconds_per_step=tot / len(times), cores=cores, samples=samples,
                 sample=f'{args.net} {args.solver} num_steps={args.num_steps} batch {args.cpu_batch} (same net/solver/NFE, bounded batch), '
                        f'{len(times)} timed + {warmup} warm-up passes, torch CPU fp32 {torch.__version__}, {cores} threads')
 
@@ -232,7 +257,9 @@ def main():
     if args.impl == 'reference':
         if rank != 0:
             return
-        cb = cpu_reference_leg(args, max(1, args.steps), min(args.warmup, 1))
+        cb = cpu_reference_leg(args, args.steps, min(args.warmup, 1))
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dict(samples=cb['samples']))
         # same net / solver / NFE as the native arm's config; each step is a BOUNDED SAMPLE of it (batch `cpu_batch`, not batch_per_gpu)
         config['workload'] += f' -- CPU arm: each step is a bounded sample of this workload, batch {args.cpu_batch} on {cb["cores"]} host threads'
         config['sample_batch'] = args.cpu_batch
@@ -289,6 +316,7 @@ def main():
     launches = net.total_launches + solver_utils.LAUNCHES[0] - l0
     clk = clocks.stop() if rank == 0 else None
     value = world * B * args.steps / (ms / 1e3)
+    dumps = dict(samples=images.cpu()) if args.dump_outputs and rank == 0 else None
 
     # ---- end-to-end through the public API with host buffers -------------------------------------------------------
     e2e = None
@@ -368,11 +396,13 @@ def main():
     if solo and args.all_configs and (args.net, args.solver) == ('cifar10', 'heun'):
         del net, images
         torch.cuda.empty_cache()
-        line['configs'] = other_configs(args, dev, pk)
+        line['configs'] = other_configs(args, dev, pk, dumps)
 
     if not args.no_cpu_baseline and world == 1:
         cb = cpu_reference_leg(args, 1, 1)
         line['cpu_baseline'] = dict(value=cb['value'], unit='images/s', cores=cb['cores'], kind='port', sample=cb['sample'])
+    if dumps:
+        write_outputs(args.dump_outputs, dumps)
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
@@ -393,9 +423,10 @@ OTHER_CONFIGS = [
 ]
 
 
-def other_configs(args, dev, pk):
+def other_configs(args, dev, pk, dumps=None):
     """BASELINE configs 3-5 on one GPU at their per-GPU batch: value (latents resident), e2e (host buffers), roofline of the GEMM
-    kernel (CUDA events per op), the eager-PyTorch comparator where the oracle has a GPU-capable net (configs 3, 4)."""
+    kernel (CUDA events per op), the eager-PyTorch comparator where the oracle has a GPU-capable net (configs 3, 4).  With `dumps`,
+    each config's last timed samples go in as config<id>_samples."""
     import copy
     import torch
     out = []
@@ -434,6 +465,8 @@ def other_configs(args, dev, pk):
             clocks.start()
             ms, images = timed_steps(step, args.config_steps, sync, dev, 1)
             ent['clocks'] = clocks.stop()
+            if dumps is not None:
+                dumps[f'config{c["id"]}_samples'] = images.cpu()
             ent['value'] = a.batch * args.config_steps / (ms / 1e3)
             ent['unit'] = 'images/s (1 GPU)'
             ent['ms_per_step'] = ms / args.config_steps
